@@ -19,6 +19,8 @@ vorticity confinement and the CNN pressure projection -- BASELINE.json configs[2
             used is stated)
 
 `--impl reference` times that CPU path alone and prints the same line shape.
+`--dump-outputs DIR` writes the state the last timed step left (pDiv, UDiv, density) as DIR/<name>.npy, float32;
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 Multi-GPU (N > 1, launched with torchrun): weak scaling -- every rank advances an
 independent 128^3 grid (the batch-of-grids decomposition north_star allows); no data-path
 collective; time = max over ranks.
@@ -46,6 +48,21 @@ ALGO_BYTES = {
     "advect_scalar": 24,    # s 4 + U 12 + flags 4 read, s 4 written
     "cnn": 36,              # pDiv 4 + UDiv 12 + flags 4 read, p 4 + U 12 written
 }
+# --dump-outputs writes at most this many bytes of array data (a 128^3 step's state is 42 MB)
+DUMP_LIMIT_BYTES = 60 * 10 ** 6
+
+
+def dump_outputs(directory, arrays):
+    """Writes each array as <directory>/<name>.npy in float32.  Above DUMP_LIMIT_BYTES in all, each array is cut
+    to a fixed, seeded sample of its flat indices, sized to its share of the limit."""
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.size * 4 for a in arrays.values())
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, np.float32)
+        if total > DUMP_LIMIT_BYTES:
+            k = a.size * DUMP_LIMIT_BYTES // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).integers(0, a.size, k))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def use_all_host_cores():
@@ -302,7 +319,11 @@ def main():
                     help="grids: one independent --grid^3 domain per GPU (weak scaling, the default and the "
                          "BASELINE metric); slab: ONE --grid^3 domain z-slab decomposed over the GPUs with NCCL "
                          "halo exchange (strong scaling, BASELINE config 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write pDiv, UDiv and density after the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.mode == "slab"):
+        ap.error("--dump-outputs applies to the default GPU measurement (--impl b200 --mode grids)")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -381,6 +402,8 @@ def main():
         except Exception as e:                      # a box that cannot capture: the kernel-by-kernel number is the headline
             graph_error = "%s: %s" % (type(e).__name__, e)
             graph_ms, graph_launches = total_ms, launches
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {k: gb[k].cpu().numpy() for k in ("pDiv", "UDiv", "density")})
         # trace-length regime of the timed steps (the advection cost is data dependent)
         max_u_dt = float(gb["UDiv"].abs().max().item()) * mconf["dt"]
         if world > 1:

@@ -32,9 +32,8 @@ def orc():
     return oracle.Oracle()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    import oracle
-    if not oracle.have_reference():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    return oracle.Reference()
+@pytest.fixture
+def ref(request):
+    """The reference's recorded outputs for this test (tests/reference_record.py)."""
+    from reference_record import RecordedReference
+    return RecordedReference("%s::%s" % (request.node.path.stem, request.node.name))

@@ -36,6 +36,23 @@ def test_reference_arm_json_line():
     assert d["cpu_baseline"]["kind"] in ("reference", "port")
 
 
+def test_dump_outputs_float32_and_a_fixed_sample_above_the_limit(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    a = np.arange(3000, dtype=np.float64).reshape(3, 10, 100)
+    bench.dump_outputs(str(tmp_path / "full"), {"U": a})
+    got = np.load(tmp_path / "full" / "U.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, a.astype(np.float32))
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4000)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"U": a, "p": a[0]})
+    s1 = {k: np.load(tmp_path / "s1" / (k + ".npy")) for k in ("U", "p")}
+    assert s1["U"].size == 750 and s1["p"].size == 250          # each array's share of the 4000 bytes
+    for k, v in s1.items():
+        assert np.array_equal(v, np.load(tmp_path / "s2" / (k + ".npy")))
+        assert np.all(np.diff(v) >= 0) and np.isin(v, a).all()
+
+
 def test_roofline_traffic_is_read_from_the_tracked_ncu_table():
     """bench.py's roofline.traffic comes from profiles/r02_advect_ncu_raw.csv (the ncu --set full capture of the
     current advection kernels), never from a literal: the parser finds the kernel and gives DRAM bytes per launch."""

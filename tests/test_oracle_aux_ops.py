@@ -1,19 +1,13 @@
 """normalizePressureMean, volumetricUpSamplingNearestForward, rectangularBlur, signedDistanceField:
-the oracle's restatements against the reference's own CPU code (oracle/_ref), bit for bit; the mean
-removal to float rounding (the reference accumulates it with an OpenMP atomic, order unspecified)."""
+the oracle's restatements against the reference's own CPU code (oracle/_ref, outputs recorded under tests/golden),
+bit for bit; the mean removal to float rounding (the reference accumulates it with an OpenMP atomic, order
+unspecified)."""
 import numpy as np
 import pytest
 
 from oracle import api
-from cases import bits_equal, describe_diff
+from cases import bits_equal
 import pcg_cases
-
-
-@pytest.fixture(scope="module")
-def ref():
-    if not api.have_reference():
-        pytest.skip("oracle/_ref not built")
-    return api.Reference()
 
 
 @pytest.fixture(scope="module")
@@ -31,18 +25,18 @@ def fields(orc, is3d, seed=0):
 def test_upsampling(orc, ref, is3d):
     _, x = fields(orc, is3d)
     x = np.ascontiguousarray(x[:, :, :5, :6, :7])
+    ref.check(orc, lambda be: {"ratio=%d" % ratio: be.volumetricUpSamplingNearestForward(ratio, x)
+                               for ratio in (1, 2, 3)})
     for ratio in (1, 2, 3):
-        a, b = orc.volumetricUpSamplingNearestForward(ratio, x), ref.volumetricUpSamplingNearestForward(ratio, x)
-        assert bits_equal(a, b)
+        a = orc.volumetricUpSamplingNearestForward(ratio, x)
         assert a.shape[2:] == tuple(s * ratio for s in x.shape[2:])
 
 
 @pytest.mark.parametrize("is3d", [True, False])
 def test_rectangular_blur(orc, ref, is3d):
     _, x = fields(orc, is3d)
-    for rad in (1, 2, 5, 40):               # 40 > every extent: the clamped-edge branches
-        a, b = orc.rectangularBlur(x, rad, is3d), ref.rectangularBlur(x, rad, is3d)
-        assert bits_equal(a, b), describe_diff(a, b)
+    # 40 > every extent: the clamped-edge branches
+    ref.check(orc, lambda be: {"rad=%d" % rad: be.rectangularBlur(x, rad, is3d) for rad in (1, 2, 5, 40)})
     const = np.full_like(x, 3.0)
     assert np.allclose(orc.rectangularBlur(const, 3, is3d), 3.0, atol=1e-5)
 
@@ -50,9 +44,9 @@ def test_rectangular_blur(orc, ref, is3d):
 @pytest.mark.parametrize("is3d", [True, False])
 def test_signed_distance_field(orc, ref, is3d):
     flags, _ = fields(orc, is3d)
+    ref.check(orc, lambda be: {"rad=%d" % rad: be.signedDistanceField(flags, rad, is3d) for rad in (1, 3)})
     for rad in (1, 3):
-        a, b = orc.signedDistanceField(flags, rad, is3d), ref.signedDistanceField(flags, rad, is3d)
-        assert bits_equal(a, b)
+        a = orc.signedDistanceField(flags, rad, is3d)
         assert np.all(a[flags == 2] == 0) and a.max() <= rad
 
 
@@ -60,11 +54,9 @@ def test_signed_distance_field(orc, ref, is3d):
 def test_normalize_pressure_mean(orc, ref, is3d):
     flags, x = fields(orc, is3d)
     flags[0, 0, 0, 3, 3] = 1                 # a fluid cell on the border is legal here
-    p1 = np.ascontiguousarray(x[:, :1]).copy()
-    p2 = p1.copy()
-    orc.normalizePressureMean(p1, flags, is3d)
-    ref.normalizePressureMean(p2, flags, is3d)
-    assert np.abs(p1 - p2).max() <= 2e-6 * np.abs(p2).max()
+    p0 = np.ascontiguousarray(x[:, :1]).copy()
+    ref.check(orc, lambda be: {"p": be.normalizePressureMean(p0.copy(), flags, is3d)}, tol={"p": 2e-6})
+    p1 = orc.normalizePressureMean(p0.copy(), flags, is3d)
     assert bits_equal(p1[flags != 1], x[:, :1][flags != 1])          # non-fluid cells untouched
     comp, sizes = orc.findConnectedFluidComponents(flags, is3d, 0)
     for ic in range(len(sizes)):
@@ -82,17 +74,19 @@ def test_backward_operators(orc, ref, is3d):
     fl = synth.make_flags(nx, ny, nz, is3d, nb=2, geometry=True, exotic=True)
     U = synth.make_velocity(fl, is3d, amp=1.0)
     go = rng.standard_normal(fl.shape).astype(np.float32)
-    a, b = orc.velocityDivergenceBackward(U, fl, go), ref.velocityDivergenceBackward(U, fl, go)
-    assert bits_equal(a, b), describe_diff(a, b)
     goU = rng.standard_normal(U.shape).astype(np.float32)
     p = rng.standard_normal(fl.shape).astype(np.float32)
-    a, b = orc.velocityUpdateBackward(U, fl, p, goU), ref.velocityUpdateBackward(U, fl, p, goU)
-    assert np.abs(a - b).max() <= 1e-6 * np.abs(b).max()
     x = rng.standard_normal((2, 3, 4, 5, 6)).astype(np.float32)
-    for ratio in (1, 2, 3):
-        g = rng.standard_normal((2, 3, 4 * ratio, 5 * ratio, 6 * ratio)).astype(np.float32)
-        assert bits_equal(orc.volumetricUpSamplingNearestBackward(ratio, x, g),
-                          ref.volumetricUpSamplingNearestBackward(ratio, x, g))
+    gs = [rng.standard_normal((2, 3, 4 * ratio, 5 * ratio, 6 * ratio)).astype(np.float32) for ratio in (1, 2, 3)]
+
+    def run(be):
+        out = {"velocityDivergenceBackward": be.velocityDivergenceBackward(U, fl, go),
+               "velocityUpdateBackward": be.velocityUpdateBackward(U, fl, p, goU)}
+        for ratio, g in zip((1, 2, 3), gs):
+            out["volumetricUpSamplingNearestBackward/ratio=%d" % ratio] = \
+                be.volumetricUpSamplingNearestBackward(ratio, x, g)
+        return out
+    ref.check(orc, run, tol={"velocityUpdateBackward": 1e-6})
 
 
 def test_backward_is_the_adjoint(orc):

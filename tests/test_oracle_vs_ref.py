@@ -1,11 +1,11 @@
 """Pins the C restatement (oracle/tfluids_oracle.c) against the reference's own CPU code
 compiled in place (oracle/_ref): bit-exact on seeded inputs for every operator and
-advection method.  Skipped where /root/reference (hence oracle/_ref) is unavailable."""
+advection method.  The reference's outputs are recorded under tests/golden (tests/reference_record.py)."""
 import numpy as np
 import pytest
 
 import oracle
-from cases import CASES, CASE_IDS, build, bits_equal, describe_diff
+from cases import CASES, CASE_IDS, build
 
 METHODS = list(oracle.ADVECT_METHODS)
 
@@ -16,10 +16,9 @@ def test_advect_scalar(orc, ref, case, method):
     c = build(case)
     U = c["U"].copy()
     orc.setWallBcsForward(U, c["flags"])
-    for outside in (False, True):
-        a = orc.advectScalar(0.1, c["density"], U, c["flags"], method, outside, 0.6)
-        b = ref.advectScalar(0.1, c["density"], U, c["flags"], method, outside, 0.6)
-        assert bits_equal(a, b), describe_diff(a, b)
+    ref.check(orc, lambda be: {"outside=%d" % outside: be.advectScalar(0.1, c["density"], U, c["flags"], method,
+                                                                       outside, 0.6)
+                               for outside in (False, True)})
     assert orc.trace_faults() == 0
 
 
@@ -29,69 +28,65 @@ def test_advect_vel(orc, ref, case, method):
     c = build(case)
     U = c["U"].copy()
     orc.setWallBcsForward(U, c["flags"])
-    a = orc.advectVel(0.1, U, c["flags"], method, 0.6)
-    b = ref.advectVel(0.1, U, c["flags"], method, 0.6)
-    assert bits_equal(a, b), describe_diff(a, b)
+    ref.check(orc, lambda be: {"advectVel": be.advectVel(0.1, U, c["flags"], method, 0.6)})
 
 
 @pytest.mark.parametrize("case", CASES, ids=CASE_IDS)
 def test_pointwise_operators(orc, ref, case):
     c = build(case)
     fl = c["flags"]
-    for mask in (False, True):
-        a, b = c["U"].copy(), c["U"].copy()
-        orc.setWallBcsForward(a, fl, mask)
-        ref.setWallBcsForward(b, fl, mask)
-        assert bits_equal(a, b), "setWallBcs " + describe_diff(a, b)
     U = c["U"].copy()
     orc.setWallBcsForward(U, fl)
-    a, b = orc.velocityDivergenceForward(U, fl), ref.velocityDivergenceForward(U, fl)
-    assert bits_equal(a, b), "divergence " + describe_diff(a, b)
-    a, b = U.copy(), U.copy()
-    orc.velocityUpdateForward(a, fl, c["p"])
-    ref.velocityUpdateForward(b, fl, c["p"])
-    assert bits_equal(a, b), "velocityUpdate " + describe_diff(a, b)
     g = [0.1, -0.7, 0.3]
-    a, b = U.copy(), U.copy()
-    orc.addBuoyancy(a, fl, c["density"], g, 0.1)
-    ref.addBuoyancy(b, fl, c["density"], g, 0.1)
-    assert bits_equal(a, b), "addBuoyancy " + describe_diff(a, b)
-    a, b = U.copy(), U.copy()
-    orc.addGravity(a, fl, g, 0.1)
-    ref.addGravity(b, fl, g, 0.1)
-    assert bits_equal(a, b), "addGravity " + describe_diff(a, b)
-    a, b = U.copy(), U.copy()
-    orc.vorticityConfinement(a, fl, 0.3)
-    ref.vorticityConfinement(b, fl, 0.3)
-    assert bits_equal(a, b), "vorticityConfinement " + describe_diff(a, b)
+
+    def run(be):
+        out = {}
+        for mask in (False, True):
+            a = c["U"].copy()
+            be.setWallBcsForward(a, fl, mask)
+            out["setWallBcs/mask=%d" % mask] = a
+        out["divergence"] = be.velocityDivergenceForward(U, fl)
+        for name, fn in (("velocityUpdate", lambda a: be.velocityUpdateForward(a, fl, c["p"])),
+                         ("addBuoyancy", lambda a: be.addBuoyancy(a, fl, c["density"], g, 0.1)),
+                         ("addGravity", lambda a: be.addGravity(a, fl, g, 0.1)),
+                         ("vorticityConfinement", lambda a: be.vorticityConfinement(a, fl, 0.3))):
+            a = U.copy()
+            fn(a)
+            out[name] = a
+        return out
+    ref.check(orc, run)
 
 
 def test_empty_domain_and_occupancy(orc, ref):
-    for is3d, shape in ((True, (2, 1, 7, 9, 11)), (False, (2, 1, 1, 9, 11))):
-        for bnd in (1, 2):
-            a = np.zeros(shape, np.float32)
-            b = np.zeros(shape, np.float32)
-            orc.emptyDomain(a, is3d, bnd)
-            ref.emptyDomain(b, is3d, bnd)
-            assert bits_equal(a, b)
-            assert bits_equal(orc.flagsToOccupancy(a), ref.flagsToOccupancy(b))
+    def run(be):
+        out = {}
+        for is3d, shape in ((True, (2, 1, 7, 9, 11)), (False, (2, 1, 1, 9, 11))):
+            for bnd in (1, 2):
+                a = np.zeros(shape, np.float32)
+                be.emptyDomain(a, is3d, bnd)
+                out["emptyDomain/%dd/bnd=%d" % (3 if is3d else 2, bnd)] = a
+                out["flagsToOccupancy/%dd/bnd=%d" % (3 if is3d else 2, bnd)] = be.flagsToOccupancy(a)
+        return out
+    ref.check(orc, run)
 
 
 def test_line_trace_random(orc, ref):
     rs = np.random.RandomState(5)
     from fluidnet_b200 import synth
     flags = synth.make_flags(20, 18, 16, True, nb=1, geometry=True)
-    n = 0
+    traces = []
     for _ in range(4000):
         pos = (rs.rand(3) * [18, 16, 14] + 1).astype(np.float32)
         if (int(flags[0, 0, int(pos[2]), int(pos[1]), int(pos[0])]) & 1) == 0:
             continue
         delta = (rs.randn(3) * rs.choice([0.3, 2.0, 9.0])).astype(np.float32)
-        ha, pa = orc.calcLineTrace(pos, delta, flags)
-        hb, pb = ref.calcLineTrace(pos, delta, flags)
-        assert ha == hb and bits_equal(pa, pb), (pos, delta, pa, pb)
-        n += 1
-    assert n > 2000
+        traces.append((pos, delta))
+    assert len(traces) > 2000
+
+    def run(be):
+        res = [be.calcLineTrace(pos, delta, flags) for pos, delta in traces]
+        return {"hit": np.array([h for h, _ in res], np.int32), "pos": np.array([p for _, p in res], np.float32)}
+    ref.check(orc, run)
 
 
 TILE_GRIDS = [((40, 24, 20), True, False), ((36, 20, 12), True, True), ((64, 16, 5), False, False)]
@@ -109,15 +104,16 @@ def test_maccormack_ours_in_the_tile_kernels_regimes(orc, ref, dims, geom, exoti
     flags = synth.make_flags(nx, ny, nz, True, nb=1, geometry=geom, exotic=exotic)
     U = synth.make_velocity(flags, True, amp=amp)
     orc.setWallBcsForward(U, flags)
-    a = orc.advectVel(0.1, U, flags, "maccormackOurs", 0.6)
-    b = ref.advectVel(0.1, U, flags, "maccormackOurs", 0.6)
-    assert bits_equal(a, b), "advectVel " + describe_diff(a, b)
     rho = synth.make_density(flags)
     rho[np.random.RandomState(3).rand(*rho.shape) < 0.3] = 0.0
-    for outside in (False, True):
-        a = orc.advectScalar(0.1, rho, U, flags, "maccormackOurs", outside, 0.6)
-        b = ref.advectScalar(0.1, rho, U, flags, "maccormackOurs", outside, 0.6)
-        assert bits_equal(a, b), "advectScalar(outside=%s) %s" % (outside, describe_diff(a, b))
+
+    def run(be):
+        out = {"advectVel": be.advectVel(0.1, U, flags, "maccormackOurs", 0.6)}
+        for outside in (False, True):
+            out["advectScalar/outside=%d" % outside] = be.advectScalar(0.1, rho, U, flags, "maccormackOurs",
+                                                                       outside, 0.6)
+        return out
+    ref.check(orc, run)
 
 
 def test_signed_zero_fields_match_the_reference(orc, ref):
@@ -130,6 +126,4 @@ def test_signed_zero_fields_match_the_reference(orc, ref):
     U[rng.rand(*U.shape) < 0.35] = 0.0
     U[rng.rand(*U.shape) < 0.2] = -0.0
     orc.setWallBcsForward(U, flags)
-    a = orc.advectVel(0.1, U, flags, "maccormackOurs", 0.6)
-    b = ref.advectVel(0.1, U, flags, "maccormackOurs", 0.6)
-    assert bits_equal(a, b), describe_diff(a, b)
+    ref.check(orc, lambda be: {"advectVel": be.advectVel(0.1, U, flags, "maccormackOurs", 0.6)})

@@ -1,17 +1,17 @@
 """fluidnet_b200/torch7.py: the Torch7 binary reader that brings a model trained with the reference into
 this library (SURVEY.md section 8f-2).  A writer for the same format lives here (test-only) so the reader
-is exercised without Torch7; the trained 2-D model the reference ships is read when /root/reference is
-present and must match the committed fixture (tests/golden/myModel2D_layers.npz)."""
+is exercised without Torch7; the trained 2-D model the reference ships (tests/golden/myModel2D_slim: the file
+with its large buffers emptied, tests/golden/make_model_fixture.py) must match the committed weights
+(tests/golden/myModel2D_layers.npz)."""
 import os
 import struct
 
 import numpy as np
-import pytest
 
 from fluidnet_b200 import torch7
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "myModel2D_layers.npz")
-REF_MODEL = "/root/reference/data/models/myModel2D"
+REF_MODEL = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "myModel2D_slim")
 
 
 class W:
@@ -98,7 +98,6 @@ def test_back_references(tmp_path):
     assert t["a"] is t["b"] and t["a"][1] == 7
 
 
-@pytest.mark.skipif(not os.path.exists(REF_MODEL), reason="/root/reference not present")
 def test_shipped_2d_model_matches_fixture():
     """The reference's trained model (nngraph gModule of cudnn.SpatialConvolution layers): 'default' 2-D
     architecture of torch/lib/model.lua:179-186, and the same numbers as the committed fixture."""
